@@ -29,6 +29,11 @@ the per-trajectory configuration is the headline C3's).  Prints ONE JSON line (r
   cpu_baseline  the CPU oracle (restatement of the reference's Eigen path, oracle/oracle.cpp)
              on all usable host cores (affinity and cgroup quota respected), bounded sample (rank 0, N=1).
 
+--dump-outputs DIR  after the timed steps, writes what the last one computed -- the coefficients and the per-trajectory
+             status of a fixed, seeded sample of the batch (32 MiB of coefficients at most) and the sampled row
+             indices -- as DIR/{coeffs,status,rows}.npy (float64; a _rank<r> suffix per rank when N > 1).  The
+             inputs depend only on the arguments, so two builds can be compared output for output.
+
 --impl reference times that CPU restatement itself (the reference needs Eigen/glog, absent
 from this image, so oracle/_ref cannot exist; see DESIGN.md): kind "port".
 """
@@ -167,6 +172,24 @@ def synth_batch(torch, N, K, D, B, device, seed):
     dfix[:, :, h:h + K - 1] = pos[:, 1:K].transpose(1, 2)
     dfix[:, :, h + K - 1] = pos[:, K]
     return pos, times.contiguous(), dfix.contiguous()
+
+
+DUMP_BYTES = 32 << 20  # coefficient bytes written by --dump-outputs
+
+
+def dump_outputs(torch, out_dir, coeffs, status, lo, total, world, rank):
+    """Writes the sampled rows of this rank's outputs (coeffs [B][K][D][N], status [B] of global rows lo..lo+B)."""
+    import numpy as np
+    row_bytes = coeffs[0].numel() * coeffs.element_size()
+    n = min(total, max(1, DUMP_BYTES // row_bytes))
+    rows = np.sort(np.random.default_rng(0).choice(total, size=n, replace=False))
+    rows = rows[(rows >= lo) & (rows < lo + coeffs.shape[0])]
+    idx = torch.from_numpy(rows - lo).to(coeffs.device)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"rows{suffix}.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, f"coeffs{suffix}.npy"), coeffs[idx].cpu().numpy())
+    np.save(os.path.join(out_dir, f"status{suffix}.npy"), status[idx].cpu().numpy().astype(np.float64))
 
 
 def _best_threads(O, N, r, K, D):
@@ -457,6 +480,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     ok = bool((status == 0).all().item()) and bool(torch.isfinite(coeffs).all().item())
     value = total * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs:  # before the phases below reuse `coeffs`
+        dump_outputs(torch, args.dump_outputs, coeffs, status, bounds[rank], total, world, rank)
 
     # ---------------- BASELINE C5 data path: root holds the batch, NCCL scatter / solve / gather
     sg = None
@@ -719,7 +744,11 @@ def main():
     ap.add_argument("--no-peer-paths", action="store_true",
                     help="skip the two NVLink peer-memory variants of the C5 data path (fused solve + gather through TMA "
                          "stores into the root's output; copy-engine pull / solve / push pipeline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed, seeded sample of the last timed step's outputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the CUDA path; the reference arm does not keep its coefficients")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -4,6 +4,7 @@
 // (value types, fixtures, static helpers, layout); without it every solve goes through the GPU.
 #include <cmath>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <iostream>
 #include <sstream>
@@ -11,6 +12,8 @@
 #include <random>
 #include <string>
 #include <vector>
+
+#include <unistd.h>
 
 #include "mav_trajectory_generation/batch_polynomial_optimization.h"
 #include "mav_trajectory_generation/io.h"
@@ -495,7 +498,13 @@ static void testTrajectorySampling() {
     EXPECT(!sampleTrajectoryInRange(t4, 0.4, t4.getMaxTime() + 1.0, dt, &states));
   }
   {  // Matlab dump of the sampled states (io.h): one row per 0.01 s sample, 27 aligned columns
-    const std::string path = "/tmp/mtg_sampled_states_test.txt";
+    // a private file (mkstemp): a fixed name in a shared temp directory may belong to another user or run
+    const char* tmpdir = std::getenv("TMPDIR");
+    std::string tmpl = std::string(tmpdir && *tmpdir ? tmpdir : "/tmp") + "/mtg_sampled_states_XXXXXX";
+    const int fd = mkstemp(&tmpl[0]);
+    EXPECT(fd >= 0);
+    if (fd >= 0) close(fd);
+    const std::string path = tmpl;
     EXPECT(sampledTrajectoryStatesToFile(path, t4));
     std::ifstream fin(path);
     std::string line;
