@@ -113,6 +113,9 @@ int mtg_device_is_sm100(const mtg_handle* h);
                                     2 (default) = also where only one fits (single buffered) */
 #define MTG_OPT_EARLY_REFILL 10   /* TMA-input kernel with one tile buffer: 0 = the buffer is refilled with the next tile two
                                    * outward-sweep steps before the tile ends (default), -1 = while the last segment is emitted */
+#define MTG_OPT_V5_STATIC_SHAPE 11 /* TMA-input kernel: 0 = the instantiation compiled for the problem's K (K = 16 and 8 at
+                                    * N = 10, r = 4, D = 3; K = 4 at N = 8, r = 3, D = 3) where the launch layout is the one
+                                    * it was built for (default), -1 = always the run-time-shape kernel; bitwise identical */
 #define MTG_OPT_DYNAMIC_TILES 5   /* persistent kernel: warps draw tiles from a global counter: 0 = auto, 1 = always, 2 = never */
 int mtg_set_option(mtg_handle* h, int key, int value);
 

@@ -20,6 +20,7 @@ OPT_GENERIC_VARIANT = 7
 OPT_MELLINGER_UNFUSED = 8
 OPT_TMA_INPUTS = 9
 OPT_EARLY_REFILL = 10
+OPT_V5_STATIC_SHAPE = 11
 
 EXPORTED_SYMBOLS = [
     "mtg_create", "mtg_destroy", "mtg_last_error", "mtg_launch_count", "mtg_device_is_sm100",

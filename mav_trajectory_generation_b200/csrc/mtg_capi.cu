@@ -51,6 +51,7 @@ struct mtg_handle {
   int waypoint_variant = 0;  // MTG_OPT_WAYPOINT_VARIANT
   int ring_depth = 3;        // MTG_OPT_RING_DEPTH (v4 kernel: cp.async input ring buffers, 2..4)
   int early_steps = 0;       // MTG_OPT_EARLY_REFILL (v5, single tile buffer): 0 = on (kV5Early steps of lead), -1 = off
+  int v5_static_shape = 0;   // MTG_OPT_V5_STATIC_SHAPE: 0 = on (compile-time-shape v5 kernel where one is built), -1 = off
   int ctas_per_sm = 0;       // MTG_OPT_CTAS_PER_SM (v4 kernel: 0 = as many as fit, 9 = one CTA per tile, not persistent)
   int stagger_us = 0;        // MTG_OPT_STAGGER_US (v4 kernel: CTA start times spread over this many microseconds)
   int tma_inputs = 2;        // MTG_OPT_TMA_INPUTS (default routing prefers the TMA-input kernel v5 when eligible)
@@ -240,9 +241,7 @@ constexpr int kV4MaxK = 8;
 
 // ---- v5: v4 with the inputs moved by TMA bulk copies (whole 16-trajectory tiles, double buffered); K <= 8
 typedef void (*V5Kernel)(const mtg::WaypointParams, const mtg::TmemLaunchV5, const CUtensorMap);
-// lead (outward-sweep steps) of the single-buffer tile refill: measured on C3 / C5-on-one-GPU / K = 14 with E = off, 1, 2, 3,
-// 4 -> 0.625 / 0.638 / 0.646 / 0.641 / 0.639 (C3), 0.657 / 0.679 / 0.690 / 0.671 / 0.663 (C5x1)  [tools/early_refill_sweep.py]
-constexpr int kV5Early = 2;
+using mtg::kV5Early;
 struct V5Entry {
   int N, R, D;
   V5Kernel fn, fn_fused;
@@ -256,6 +255,24 @@ const V5Entry kV5Kernels[] = {MTG_V5(10, 4, 3, 2), MTG_V5(8, 3, 3, 3),  MTG_V5(1
 const V5Entry* find_v5(const mtg_problem* p) {
   for (const auto& e : kV5Kernels)
     if (e.N == p->N && e.R == p->r && e.D == p->D) return &e;
+  return nullptr;
+}
+// compile-time-shape instantiations (KC = K) of the v5 kernel, each built for the layout v5_static_layout() gives it
+struct V5StaticEntry {
+  int N, R, D, K;
+  V5Kernel fn;
+  mtg::V5Layout layout;
+  int early;
+};
+#define MTG_V5K(N_, R_, D_, MB_, K_)                                                                               \
+  {N_, R_, D_, K_,                                                                                                 \
+   mtg::twisted_tmem_v5_kernel<N_, R_, D_, MB_, false,                                                           \
+                               mtg::v5_static_layout<N_, D_, MB_, K_>().early_fits ? kV5Early : 0, K_>,          \
+   mtg::v5_static_layout<N_, D_, MB_, K_>(), mtg::v5_static_layout<N_, D_, MB_, K_>().early_fits ? kV5Early : 0}
+const V5StaticEntry kV5StaticKernels[] = {MTG_V5K(10, 4, 3, 2, 16), MTG_V5K(10, 4, 3, 2, 8), MTG_V5K(8, 3, 3, 3, 4)};
+const V5StaticEntry* find_v5_static(const mtg_problem* p) {
+  for (const auto& e : kV5StaticKernels)
+    if (e.N == p->N && e.R == p->r && e.D == p->D && e.K == p->K) return &e;
   return nullptr;
 }
 
@@ -684,38 +701,15 @@ int launch_solve(mtg_handle* h, const mtg_problem* p, CachedTopology* topo, int6
       const V5Entry* e5 = find_v5(p);
       if (e5) {
         const V5Kernel fn5 = fused ? e5->fn_fused : e5->fn;
-        const int hh = p->N / 2, mm = hh - 1;
-        const int kslots = mm * (mm + 1) / 2 + mm * p->D;  // no positions in the v5 state
-        const int nmax = (p->K + 1) / 2 - 1;
-        const int total_state = nmax * kslots;
         int n_regs = 0;
         {
           const int rc_regs = kernel_regs(h, (const void*)fn5, &n_regs);
           if (rc_regs != MTG_OK) return rc_regs;
         }
         const int by_regs = std::max(1, 65536 / (std::max(n_regs, 1) * mtg::kTmemThreads));
-        int best_ctas = 0, best_cols = 0, best_nbuf = 0;
-        size_t best_smem = 0;
-        const int col_options[] = {256, 128, 64, 32, 512};
-        for (int nbuf = 2; nbuf >= 1; --nbuf)
-          for (int cols : col_options) {
-            const int tslots = cols / 2;
-            const int spill = std::max(0, total_state - tslots);
-            const size_t tile_doubles = fused ? size_t(16) * (p->K + 1) * p->D : size_t(16) * (p->K + p->D * L.n_fixed);
-            const size_t smem = mtg::kTmemHeaderBytes + size_t(4) * e->stage_bytes_per_warp + 128 +
-                                size_t(4) * nbuf * tile_doubles * 8 +
-                                size_t(spill + (fused ? nmax + 1 : 0)) * mtg::kTmemThreads * 8;
-            if (smem > h->smem_optin) continue;
-            int ctas = std::min<int>(by_regs, int((228 * 1024) / (smem + 1024)));
-            ctas = std::min(std::min(ctas, 512 / cols), 8);
-            // more resident CTAs first; then double buffering; then less shared memory
-            if (ctas > best_ctas || (ctas == best_ctas && ctas > 0 && (nbuf > best_nbuf || (nbuf == best_nbuf && smem < best_smem)))) {
-              best_ctas = ctas;
-              best_cols = cols;
-              best_nbuf = nbuf;
-              best_smem = smem;
-            }
-          }
+        const mtg::V5Layout lay = mtg::v5_layout(p->N, p->D, p->K, L.n_fixed, fused != nullptr, h->smem_optin, by_regs);
+        const int best_ctas = lay.ctas, best_cols = lay.cols, best_nbuf = lay.nbuf;
+        const size_t best_smem = lay.smem;
         const bool take = best_ctas >= 2 && (h->waypoint_variant == 6 || best_nbuf == 2 || h->tma_inputs == 2);
         if (take) {
           mtg::TmemLaunchV5 tl;
@@ -724,19 +718,27 @@ int launch_solve(mtg_handle* h, const mtg_problem* p, CachedTopology* topo, int6
           tl.n_buffers = best_nbuf;
           tl.tile_counter = nullptr;
           V5Kernel launch_fn = fn5;
-          if (best_nbuf == 1 && h->early_steps >= 0) {
-            // early refill of the single tile buffer (EARLY instantiation): both lanes must own >= E vertices and the
-            // parking area must lie in tensor memory behind the state blocks still needed
-            const int E = kV5Early;
-            const int own_min = p->K - (p->K + 1) / 2 - 1;
-            const int stash = (p->D + 1) * E + p->D + mm * p->D + 1;
+          int early = 0;
+          if (h->early_steps >= 0 && lay.early_fits) {  // early refill of the single tile buffer (EARLY instantiation)
             const V5Kernel fe = fused ? e5->fn_fused_early : e5->fn_early;
-            if (fe != nullptr && E <= own_min && E <= nmax && E * kslots + stash <= best_cols / 2) {
+            if (fe != nullptr) {
               int regs_e = 0;
               const int rc_regs = kernel_regs(h, (const void*)fe, &regs_e);
               if (rc_regs != MTG_OK) return rc_regs;
-              if (65536 / (std::max(regs_e, 1) * mtg::kTmemThreads) >= best_ctas) launch_fn = fe;
+              if (65536 / (std::max(regs_e, 1) * mtg::kTmemThreads) >= best_ctas) {
+                launch_fn = fe;
+                early = kV5Early;
+              }
             }
+          }
+          // the compile-time-shape instantiation of this K, when it was built for exactly this layout
+          const V5StaticEntry* es = (h->v5_static_shape >= 0 && !fused) ? find_v5_static(p) : nullptr;
+          if (es != nullptr && es->layout.cols == best_cols && es->layout.nbuf == best_nbuf && es->early == early &&
+              L.n_fixed == p->K + p->N - 1) {
+            int regs_s = 0;
+            const int rc_regs = kernel_regs(h, (const void*)es->fn, &regs_s);
+            if (rc_regs != MTG_OK) return rc_regs;
+            if (65536 / (std::max(regs_s, 1) * mtg::kTmemThreads) >= best_ctas) launch_fn = es->fn;
           }
           const int64_t blocks = std::min<int64_t>((B + 63) / 64, int64_t(best_ctas) * h->sm_count);
           // dynamic tile counter for long tiles with several tiles per warp (balances the tail: C3 0.618 vs 0.605,
@@ -1083,6 +1085,10 @@ int mtg_set_option(mtg_handle* h, int key, int value) {
   }
   if (key == MTG_OPT_EARLY_REFILL && value >= -1 && value <= 0) {
     h->early_steps = value;
+    return MTG_OK;
+  }
+  if (key == MTG_OPT_V5_STATIC_SHAPE && value >= -1 && value <= 0) {
+    h->v5_static_shape = value;
     return MTG_OK;
   }
   if (key == MTG_OPT_RING_DEPTH && value >= 2 && value <= 4) {

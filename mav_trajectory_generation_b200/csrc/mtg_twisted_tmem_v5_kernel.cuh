@@ -32,19 +32,19 @@ struct TmemLaunchV5 {
 };
 
 // sweep state per eliminated vertex: L (strictly lower) + inverse pivots + y  (positions come from the input tile)
-template <int N, int D>
-__host__ __device__ constexpr int v5_state_slots() {
-  constexpr int m = N / 2 - 1;
-  return m * (m + 1) / 2 + m * D;
+__host__ __device__ constexpr int v5_state_slots(int N, int D) {
+  return (N / 2 - 1) * (N / 2) / 2 + (N / 2 - 1) * D;
 }
-// dynamic shared memory: [holder 128][staging x 4 warps][mbarriers 128][input tiles: 4 warps x nbuf x 16*(K + D*nf)][spill]
-template <int N, int D>
-__host__ __device__ constexpr size_t v5_smem_bytes(int K, int nf, int tmem_slots, int nbuf) {
+// dynamic shared memory: [holder 128][staging x 4 warps][mbarriers 128][input tiles: 4 warps x nbuf x tile][spill]
+// [FUSED: segment-time history]; a tile is 16*(K + D*nf) doubles (FUSED: the waypoints, 16*(K+1)*D)
+__host__ __device__ constexpr size_t v5_smem_bytes(int N, int D, int K, int nf, int tmem_slots, int nbuf, bool fused) {
   const int nmax = (K + 1) / 2 - 1;
-  const int total = nmax * v5_state_slots<N, D>();
+  const int total = nmax * v5_state_slots(N, D);
   const int spill = total > tmem_slots ? total - tmem_slots : 0;
-  return size_t(kTmemHeaderBytes) + size_t(kTmemThreads / 32) * tmem_stage_bytes_per_warp<N, D>() + 128 +
-         size_t(kTmemThreads / 32) * nbuf * 16 * size_t(K + D * nf) * 8 + size_t(spill) * kTmemThreads * 8;
+  const size_t tile_doubles = fused ? size_t(16) * (K + 1) * D : size_t(16) * (K + D * nf);
+  const size_t stage_bytes_per_warp = size_t(32) * D * (N / 2) * 16;  // tmem_stage_bytes_per_warp<N, D>()
+  return size_t(kTmemHeaderBytes) + size_t(kTmemThreads / 32) * stage_bytes_per_warp + 128 +
+         size_t(kTmemThreads / 32) * nbuf * tile_doubles * 8 + size_t(spill + (fused ? nmax + 1 : 0)) * kTmemThreads * 8;
 }
 
 namespace bulk {
@@ -80,14 +80,70 @@ __device__ __forceinline__ void copy_g2s(uint32_t dst, const void* src, uint32_t
 // state blocks that are already popped (blocks >= E), and the tile buffer is refilled with the next tile there and
 // then: E back-substitution + emission steps of lead for the fetch instead of one.  The host launches this
 // instantiation only when n_buffers == 1, both lanes own >= E vertices, and the parking area lies inside tensor memory.
-template <int N, int D>
-__host__ __device__ constexpr int v5_early_stash_slots(int E) {
+__host__ __device__ constexpr int v5_early_stash_slots(int N, int D, int E) {
   return (D + 1) * E + D + (N / 2 - 1) * D + 1;
 }
+// lead (outward-sweep steps) of the single-buffer tile refill: measured on C3 / C5-on-one-GPU / K = 14 with E = off, 1, 2, 3,
+// 4 -> 0.625 / 0.638 / 0.646 / 0.641 / 0.639 (C3), 0.657 / 0.679 / 0.690 / 0.671 / 0.663 (C5x1)  [tools/early_refill_sweep.py]
+constexpr int kV5Early = 2;
 
-template <int N, int R, int D, int MINB, bool FUSED = false, int EARLY = 0>
+// Launch layout of the v5 kernel for one shape: tensor-memory columns, input tile buffers, dynamic shared memory and
+// resident CTAs per SM, and whether the early refill's parking area fits (single buffer only).  The host searches it at
+// run time (smem_optin of the device, by_regs = CTAs per SM the kernel's registers allow); the compile-time-shape
+// instantiations (KC > 0) are compiled for the result of the same search at the B200's budget.
+struct V5Layout {
+  int ctas = 0, cols = 0, nbuf = 0;
+  size_t smem = 0;
+  bool early_fits = false;
+};
+__host__ __device__ constexpr V5Layout v5_layout(int N, int D, int K, int nf, bool fused, size_t smem_optin, int by_regs) {
+  const int nmax = (K + 1) / 2 - 1;
+  V5Layout best{};
+  const int col_options[] = {256, 128, 64, 32, 512};
+  for (int nbuf = 2; nbuf >= 1; --nbuf)
+    for (int cols : col_options) {
+      const size_t smem = v5_smem_bytes(N, D, K, nf, cols / 2, nbuf, fused);
+      if (smem > smem_optin) continue;
+      int ctas = int((228 * 1024) / (smem + 1024));
+      ctas = by_regs < ctas ? by_regs : ctas;
+      ctas = 512 / cols < ctas ? 512 / cols : ctas;
+      ctas = ctas < 8 ? ctas : 8;
+      // more resident CTAs first; then double buffering; then less shared memory
+      if (ctas > best.ctas ||
+          (ctas == best.ctas && ctas > 0 && (nbuf > best.nbuf || (nbuf == best.nbuf && smem < best.smem)))) {
+        best.ctas = ctas;
+        best.cols = cols;
+        best.nbuf = nbuf;
+        best.smem = smem;
+      }
+    }
+  // early refill: both lanes must own >= E vertices and the parking area must lie in tensor memory behind the state
+  // blocks still needed
+  const int own_min = K - (K + 1) / 2 - 1;
+  best.early_fits = best.nbuf == 1 && kV5Early <= own_min && kV5Early <= nmax &&
+                    kV5Early * v5_state_slots(N, D) + v5_early_stash_slots(N, D, kV5Early) <= best.cols / 2;
+  return best;
+}
+// the layout a compile-time-shape instantiation is built for: waypoint constraints (n_fixed = K + N - 1), the B200's
+// 227 KB of opt-in shared memory per block, and the CTAs per SM its __launch_bounds__ guarantee
+constexpr size_t kV5StaticSmemOptin = 227 * 1024;
+template <int N, int D, int MINB, int KC>
+__host__ __device__ constexpr V5Layout v5_static_layout() {
+  return v5_layout(N, D, KC, KC + N - 1, false, kV5StaticSmemOptin, MINB);
+}
+
+// KC > 0: the instantiation for K = KC segments (waypoint constraints, no FUSED) and the launch layout
+// v5_static_layout<N, D, MINB, KC>(), which the host launches only when its run-time layout is that one.  Every shape
+// quantity is then a compile-time constant: loop trip counts, tile offsets, the TMEM / shared-memory split test of each
+// state slot, and the warp-uniform `v <= nh` tests, which vanish (K even: both lanes own K/2 - 1 vertices).
+// The arithmetic is the same expressions in the same order: results are bitwise identical to KC = 0.
+template <int N, int R, int D, int MINB, bool FUSED = false, int EARLY = 0, int KC = 0>
 __global__ void __launch_bounds__(kTmemThreads, MINB)
     twisted_tmem_v5_kernel(const WaypointParams prm, const TmemLaunchV5 tl, const __grid_constant__ CUtensorMap tmap) {
+  static_assert(KC == 0 || (!FUSED && KC % 2 == 0 && KC >= 4), "compile-time shapes: waypoint inputs, even K >= 4");
+  constexpr V5Layout kS = KC > 0 ? v5_static_layout<N, D, MINB, KC>() : V5Layout{};
+  static_assert(KC == 0 || (kS.ctas >= 2 && EARLY == (kS.early_fits ? kV5Early : 0)),
+                "compile-time shape without a v5 layout, or EARLY differs from the layout's");
   constexpr int h = N / 2;
   constexpr int m = h - 1;
   constexpr int kL = m * (m + 1) / 2;
@@ -103,13 +159,14 @@ __global__ void __launch_bounds__(kTmemThreads, MINB)
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   const int half = lane & 1;
-  const int K = prm.K;
-  const int nf = prm.n_fixed;
+  const int K = KC > 0 ? KC : prm.K;
+  const int nf = KC > 0 ? KC + N - 1 : prm.n_fixed;
   const int M = (K + 1) >> 1;
   const int nh = half ? K - M - 1 : M - 1;
   const int nmax = M - 1;
-  const int tslots = tl.tmem_slots;
-  const int nbuf = tl.n_buffers;
+  const int tslots = KC > 0 ? kS.cols / 2 : tl.tmem_slots;
+  const int tcols = KC > 0 ? kS.cols : tl.tmem_cols;
+  const int nbuf = KC > 0 ? kS.nbuf : tl.n_buffers;
 
   uint32_t* holder = reinterpret_cast<uint32_t*>(smem_raw);
   double2* stage = reinterpret_cast<double2*>(smem_raw + kTmemHeaderBytes) + size_t(warp) * 32 * (D * h);
@@ -129,8 +186,8 @@ __global__ void __launch_bounds__(kTmemThreads, MINB)
   auto SPG = [&](int s_global) -> double& { return spill[size_t(s_global - tslots) * kTmemThreads]; };
 
   uint32_t tbase = 0;
-  if (tl.tmem_cols > 0) {
-    if (warp == 0) tmem::alloc(tmem::smem_u32(holder), (uint32_t)tl.tmem_cols);
+  if (tcols > 0) {
+    if (warp == 0) tmem::alloc(tmem::smem_u32(holder), (uint32_t)tcols);
     tmem::fence_before_sync();
     __syncthreads();
     tmem::fence_after_sync();
@@ -250,13 +307,21 @@ __global__ void __launch_bounds__(kTmemThreads, MINB)
     const double* __restrict__ tT = tiles + size_t(buf) * tile_doubles + tl_row * K;
     const double* __restrict__ tF =
         tiles + size_t(buf) * tile_doubles + tile_t + tl_row * (FUSED ? (K + 1) * D : D * nf);
+    // KC > 0: own segment j and own interior vertex v (1 <= v <= K - 1) are at a per-lane base pointer plus a +-1 stride
+    // (the mirrored lane walks the tile backwards) instead of a mirrored index selected at every read
+    const int dir = half ? -1 : 1;
+    const double* tTj = tT + (half ? K - 1 : 0);
+    const double* tXv = tF + (half ? h + K - 1 : h - 1);
+    const double* tX0 = tF + (half ? h + K - 1 : 0);
     // time of own segment j: from the tile, or (FUSED) from the history filled by the inward sweep
     auto in_T = [&](int j) -> double {
       if constexpr (FUSED) return TH(j);
+      if constexpr (KC > 0) return tTj[dir * j];
       return tT[seg(j)];
     };
     auto in_x = [&](int v, int d) -> double {
       if constexpr (FUSED) return tF[(half ? K - v : v) * D + d];
+      if constexpr (KC > 0) return v == 0 ? tX0[d * nf] : tXv[d * nf + dir * v];
       return tF[d * nf + pidx(v)];
     };
     auto in_u0 = [&](int b, int d) -> double {  // fixed end derivative b+1 of own vertex 0, own-frame sign
@@ -367,6 +432,10 @@ __global__ void __launch_bounds__(kTmemThreads, MINB)
     }
 
     // ---------------------------------------------------------------- sweep towards the middle
+    // The vertex loops stay rolled also at a compile-time trip count (KC > 0): on C5 the KC = 16 kernel gains 15 % over
+    // the run-time kernel rolled (2 250 instructions), 7 % unrolled by two (4 080) and 4 % unrolled fully (7 300)
+    // (profiles/r03_v5_static_shape_variants.log): the unrolled code no longer fits the instruction caches.
+#pragma unroll 1
     for (int v = 1; v <= nmax; ++v) {
       double sv[kSlots];
       if (v <= nh) {
@@ -577,6 +646,7 @@ __global__ void __launch_bounds__(kTmemThreads, MINB)
       const uint32_t w[2] = {(uint32_t)__double2loint(val), (uint32_t)__double2hiint(val)};
       tmem::st<2>(tbase + uint32_t(2 * (kStash0 + slot)), w);
     };
+#pragma unroll 1
     for (int v = nmax; v >= 1; --v) {
       if constexpr (EARLY > 0) {
         if (v == EARLY) {
@@ -726,10 +796,10 @@ __global__ void __launch_bounds__(kTmemThreads, MINB)
   }
 
   if (lane == 0) bulk_wait_all();
-  if (tl.tmem_cols > 0) {
+  if (tcols > 0) {
     tmem::fence_before_sync();
     __syncthreads();
-    if (warp == 0) tmem::dealloc(*holder, (uint32_t)tl.tmem_cols);
+    if (warp == 0) tmem::dealloc(*holder, (uint32_t)tcols);
   }
 }
 
